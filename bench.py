@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline measurement of the B200 speculative parallel Huffman decoder.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): decoded GB/s, device-timed, on the synthetic English-like
@@ -31,6 +31,9 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 SEED = 0x48554646  # "HUFF"
+TIMING_RING = 4096   # most steps hb_ctx_timing_begin keeps per-kernel events for
+DUMP_SAMPLE = 1 << 21    # decoded bytes sampled by --dump-outputs (fixed positions, SEED)
+DUMP_BLOCK = 1 << 20     # --dump-outputs sums the decoded bytes per block of this many
 PEER = {"on": False, "seq": 0}   # map exchange by peer stores (hb_shard_exchange); seq advances on every rank alike
 WORKLOADS = {
     # name: (model kind, log2 symbols, default scaling, description).  weak: that many symbols
@@ -256,6 +259,31 @@ class Job:
         assert int(tot[0]) == self.n_total and int(tot[1]) == 0, \
             f"{self.name}: {what} mismatch: {tot.tolist()} vs {self.n_total} symbols"
 
+    def dump_outputs(self, out_dir):
+        """What the last step left for its caller, as DIR/<name>.npy (float32 / float64, about 25 MB):
+        n_symbols [symbols decoded, output base in the stream], decoded_sample (bytes at DUMP_SAMPLE
+        positions drawn with SEED, positions in decoded_sample_index) and decoded_block_sums (sum of
+        every DUMP_BLOCK bytes, so that a difference anywhere in the output shows).  The symbol count
+        is the verified first step's: every step decodes the same stream.  Ranks > 1 add _rank<r>."""
+        np, torch = self.np, self.torch
+        n = int(self.n_mine)
+        out = self.out[:n]
+        idx = np.sort(np.random.default_rng(SEED).integers(0, n, size=min(n, DUMP_SAMPLE)))
+        whole = n // DUMP_BLOCK * DUMP_BLOCK
+        sums = out[:whole].view(-1, DUMP_BLOCK).sum(dim=1, dtype=torch.int64)
+        if whole < n:
+            sums = torch.cat([sums, out[whole:].sum(dtype=torch.int64).view(1)])
+        arrays = {
+            "n_symbols": np.array([n, self.out_base], dtype=np.float64),
+            "decoded_sample": out[torch.from_numpy(idx).to(self.dev)].cpu().numpy().astype(np.float32),
+            "decoded_sample_index": idx.astype(np.float64),
+            "decoded_block_sums": sums.cpu().numpy().astype(np.float64),
+        }
+        os.makedirs(out_dir, exist_ok=True)
+        suffix = f"_rank{self.rank}" if self.world > 1 else ""
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
     def step(self, want_result=False):
         hb, c = self.hb, self.comp
         if self.world == 1:    # one GPU, one shard: the single-GPU entry point
@@ -294,7 +322,7 @@ class Job:
         self.barrier()
         if sampler is not None:
             sampler.start()
-        self.ctx.timing_begin(steps)
+        self.ctx.timing_begin(min(steps, TIMING_RING))   # per-kernel split over the first TIMING_RING steps
         e0 = torch.cuda.Event(enable_timing=True)
         e1 = torch.cuda.Event(enable_timing=True)
         self.barrier()
@@ -360,7 +388,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one decoded as DIR/<name>.npy "
+                         "(a fixed sample, block sums and the symbol count) to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path decoded")
     if args.warmup < 3:
         args.warmup = 3   # timing rule: at least three warm-up steps
     kind, log2n, dflt_scaling, desc = WORKLOADS[args.workload]
@@ -418,6 +453,8 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     ms_step, phases, (w0, w1) = job.timed(args.steps, args.warmup, sampler)
     clocks = sampler.stop(w0, w1) if rank == 0 else None
+    if args.dump_outputs:
+        job.dump_outputs(args.dump_outputs)     # before the e2e leg reuses job.out
     value = n_total / (ms_step * 1e-3) / 1e9
     in_gbs = job.nbytes_total / (ms_step * 1e-3) / 1e9
 

@@ -2,13 +2,15 @@
 
 * ``oracle/liboracle.so``  -- this repo's plain-C restatement (oracle/huff_oracle.c)
 * ``oracle/_ref/libref.so`` -- the UNMODIFIED reference CPU sources compiled by
-  ``make -C oracle ref`` in the build container (absent => those tests skip)
+  ``make -C oracle ref`` where the reference is present (absent => the tests compare
+  with the reference's recorded results instead, or skip where none are recorded)
 
 Nothing under huffmandecoderongpus_b200/ imports this module.
 """
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import hashlib
 import os
 import subprocess
@@ -64,7 +66,7 @@ def corpus_path(name: str) -> str | None:
 
 
 def plaintext_path(name: str) -> str | None:
-    fn = CORPORA[name][1]
+    fn = CORPORA[name][1] if name in CORPORA else None
     if fn is None:
         return None
     for d in (FILES_DIR, GOLDEN_DIR):
@@ -76,6 +78,32 @@ def plaintext_path(name: str) -> str | None:
 
 def sha256(buf) -> str:
     return hashlib.sha256(memoryview(np.ascontiguousarray(buf))).hexdigest()
+
+
+# Stand-in streams (not reference data).  The six larger corpora are not part of the
+# repository, so the cases that need a large stream also run on streams of the bundled
+# generator's models, built on the CPU from a fixed seed; the generated symbols are the
+# output a decode must give.  name: (model kind, symbols), sized like the corpora.
+STANDIN_SEED = 0x5354414E  # "STAN"
+STANDINS = {
+    "english4m": (0, 4047392),   # English-like order-0 text, as many symbols as bible.txt
+    "dna4m": (2, 4638690),       # four symbols of 2-bit codes, as many as E.coli
+    "fib1m": (1, 1 << 20),       # 256 symbols, codes of up to 24 bits
+    "uniform1m": (3, 1 << 20),   # eight symbols of 3-bit codes (an odd common length factor)
+}
+
+
+@functools.lru_cache(maxsize=None)
+def standin(name: str):
+    """(huffmandecoderongpus_b200.HuffFile, generated symbols) of a stand-in stream"""
+    import huffmandecoderongpus_b200 as hb
+    kind, n = STANDINS[name]
+    return hb.Model(kind).huff_file_cpu(STANDIN_SEED, n)
+
+
+def digest(name: str) -> str:
+    """SHA-256 of what decoding a corpus or a stand-in must give"""
+    return CORPORA[name][2] if name in CORPORA else sha256(standin(name)[1])
 
 
 class OraNode(C.Structure):

@@ -30,10 +30,17 @@ def ctx(dev):
 
 
 def _stream(name):
+    if name in O.STANDINS:
+        return O.standin(name)[0]
     p = O.corpus_path(name)
     if p is None:
         pytest.skip(f"{name} corpus not present")
     return hb.HuffFile.load(p)
+
+
+def _large_text():
+    """kjv where the corpus is present, else the English-like stand-in of about the same size"""
+    return "kjv" if O.corpus_path("kjv") is not None else "english4m"
 
 
 def _to_dev(data: np.ndarray, nbytes: int, dev, extra=0):
@@ -54,15 +61,18 @@ def _decode_dev(ctx, cb, f, dev, bits=None, cap=None, out_offset=0):
     return out[: res["n_symbols"]].cpu().numpy(), res, raw
 
 
-@pytest.mark.parametrize("name", list(O.CORPORA))
+@pytest.mark.parametrize("name", list(O.CORPORA) + list(O.STANDINS))
 def test_corpora_host_buffers(ctx, name):
     """BASELINE configs 1-3: every shipped corpus through hb_decode_host (upload,
-    decode, download), byte-exact against the reference's own output digest."""
+    decode, download), byte-exact against the reference's own output digest; the
+    stand-in streams against their generated symbols."""
     f = _stream(name)
     out = np.zeros(f.usize + 3, dtype=np.uint8)
     res = hb.decode_host(ctx, f.tree, f.data, f.bits, out[: f.usize])
-    assert res["n_symbols"] == f.usize == O.CORPORA[name][4]
-    assert O.sha256(out[: f.usize]) == O.CORPORA[name][2]
+    assert res["n_symbols"] == f.usize
+    if name in O.CORPORA:
+        assert f.usize == O.CORPORA[name][4]
+    assert O.sha256(out[: f.usize]) == O.digest(name)
     assert res["launches"] > 0 and res["ms_total"] > 0
     pt = O.plaintext_path(name)
     if pt is not None:
@@ -70,7 +80,9 @@ def test_corpora_host_buffers(ctx, name):
 
 
 @pytest.mark.parametrize("name,chunk", [("kjv", 64 << 10), ("kjv", 1 << 20), ("ecoli", 200000),
-                                        ("world192", 8192), ("paper1", 8192)])
+                                        ("world192", 8192), ("paper1", 8192),
+                                        ("english4m", 64 << 10), ("english4m", 1 << 20), ("dna4m", 200000),
+                                        ("fib1m", 8192), ("uniform1m", 8192)])
 def test_host_path_pipelined_chunks(dev, name, chunk):
     """hb_decode_host on streams longer than two chunks: byte-range chunks on one
     GPU with overlapped upload / decode / download, pinned and pageable buffers."""
@@ -87,7 +99,7 @@ def test_host_path_pipelined_chunks(dev, name, chunk):
             data, out = f.data, np.zeros(f.usize + 16, dtype=np.uint8)
         res = hb.decode_host(c, f.tree, data, f.bits, out[: f.usize])
         assert res["n_symbols"] == f.usize
-        assert O.sha256(out[: f.usize]) == O.CORPORA[name][2]
+        assert O.sha256(out[: f.usize]) == O.digest(name)
         assert not out[f.usize:].any()
     with pytest.raises(hb.HuffError) as e:
         hb.decode_host(c, f.tree, f.data, f.bits, np.zeros(f.usize - 1, dtype=np.uint8))
@@ -100,8 +112,8 @@ def test_host_path_pipelined_short_last_chunk_and_cut_codeword(dev):
     count bits (nor read bytes) past the end of the stream.  The stream is also cut inside a
     codeword and decoded twice into a context whose cached device buffer holds the bytes of a
     LONGER earlier decode behind the new end: the cut-off codeword must emit nothing."""
-    f = _stream("kjv")
-    st = O.load_huff(O.corpus_path("kjv"))
+    f = _stream(_large_text())
+    st = O.Stream(f.tree, f.data, f.bits, f.usize)
     chunk = 65536
     c = hb.Context(0)
     c.set_host_chunk(chunk)
@@ -123,7 +135,8 @@ def test_host_path_pipelined_short_last_chunk_and_cut_codeword(dev):
 def test_shard_host_halves_match_oracle(dev):
     """hb_shard_map_host / hb_shard_emit_host: the rank-local halves with host buffers, here for
     two shards decoded one after the other on one GPU (the exchange done by hand)"""
-    f = _stream("kjv")
+    name = _large_text()
+    f = _stream(name)
     c = hb.Context(0, stream=torch.cuda.current_stream().cuda_stream)
     cb = hb.Codebook(c, f.tree)
     nbytes = f.nbytes
@@ -153,12 +166,12 @@ def test_shard_host_halves_match_oracle(dev):
         outs.append(h_out[: res["n_symbols"]].copy())
         assert res["out_base"] == (0 if r == 0 else outs[0].size)
     got = np.concatenate(outs)
-    assert got.size == f.usize and O.sha256(got) == O.CORPORA["kjv"][2]
+    assert got.size == f.usize and O.sha256(got) == O.digest(name)
     cb.close()
     c.close()
 
 
-@pytest.mark.parametrize("name", ["hello", "paper1", "news", "book2", "kjv"])
+@pytest.mark.parametrize("name", ["hello", "paper1", "news", "book2", "kjv", "english4m", "dna4m"])
 def test_approach_drop_in(name):
     """The bigtable suite (framework/mainrun.c:541-588) calling convention:
     reference-layout structs, zeroed usize+3 output, 1 checked + repeated runs
@@ -174,13 +187,13 @@ def test_approach_drop_in(name):
 
 
 @pytest.mark.parametrize("wpt", [4, 8, 16])
-@pytest.mark.parametrize("name", ["hello", "paper1", "world192", "kjv", "ecoli"])
+@pytest.mark.parametrize("name", ["hello", "paper1", "world192", "kjv", "ecoli", "english4m", "dna4m", "fib1m", "uniform1m"])
 def test_device_resident_all_shapes(dev, name, wpt):
     f = _stream(name)
     c = hb.Context(0, stream=torch.cuda.current_stream().cuda_stream, words_per_thread=wpt)
     cb = hb.Codebook(c, f.tree)
     got, res, _ = _decode_dev(c, cb, f, dev)
-    assert got.size == f.usize and O.sha256(got) == O.CORPORA[name][2]
+    assert got.size == f.usize and O.sha256(got) == O.digest(name)
     cb.close()
     c.close()
 
@@ -276,7 +289,9 @@ def test_word_store_kernels_edge_cases(dev, path):
 
 @pytest.mark.parametrize("name,nshards,path", [("paper1", 3, "auto"), ("kjv", 2, "auto"), ("kjv", 8, "auto"),
                                                ("ecoli", 4, "auto"), ("kjv", 3, "words32w"), ("paper1", 2, "words32w"),
-                                               ("kjv", 2, "words32")])
+                                               ("kjv", 2, "words32"), ("english4m", 2, "auto"), ("english4m", 8, "auto"),
+                                               ("dna4m", 4, "auto"), ("english4m", 3, "words32w"), ("english4m", 2, "words32"),
+                                               ("fib1m", 5, "auto"), ("uniform1m", 3, "auto")])
 def test_byte_range_shards_on_one_gpu(dev, name, nshards, path):
     """The multi-GPU decomposition with every 'rank' run on cuda:0: one context
     per rank, maps gathered by concatenation, hb_shard_compose, independent emit."""
@@ -376,7 +391,7 @@ def test_full_size_round_trip(dev, kind, log2n, wpt):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("wpt", [4, 8, 16])
-@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "bible"])
+@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "bible", "english4m", "dna4m", "fib1m", "uniform1m"])
 def test_sync_paths_agree(dev, name, wpt):
     """The transducer sync kernel (default on full tiles) and the probe sync kernel
     must give the same bytes, symbol count and shard map."""
@@ -396,7 +411,7 @@ def test_sync_paths_agree(dev, name, wpt):
         outs.append((got, res["n_symbols"], res["launches"], d_map.cpu().numpy().copy()))
         cb.close()
         c.close()
-    assert O.sha256(outs[0][0]) == O.CORPORA[name][2]
+    assert O.sha256(outs[0][0]) == O.digest(name)
     for k in (1, 2, 3, 4):
         assert outs[0][1] == outs[k][1] == f.usize
         assert np.array_equal(outs[0][0], outs[k][0])
@@ -428,7 +443,7 @@ def test_hard_codes(dev, lengths, wpt):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("wpt", [4, 8, 16])
-@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "ecoli"])
+@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "ecoli", "english4m", "dna4m", "fib1m", "uniform1m"])
 def test_emit_paths_agree(dev, name, wpt):
     """word-granular staging stores (E64-table, default where the code length allows) and
     byte stores (E-table) give the same bytes, at every output alignment"""
@@ -447,19 +462,20 @@ def test_emit_paths_agree(dev, name, wpt):
         cb = hb.Codebook(c, f.tree)
         for off in (0, 1, 2, 3, 7):
             got, res, raw = _decode_dev(c, cb, f, dev, out_offset=off)
-            assert res["n_symbols"] == f.usize and O.sha256(got) == O.CORPORA[name][2], (path, off)
+            assert res["n_symbols"] == f.usize and O.sha256(got) == O.digest(name), (path, off)
             assert not raw[off + f.usize:].any() and not raw[:off].any()
         cb.close()
         c.close()
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", ["hello", "paper1", "world192", "ecoli", "fib", "english"])
+@pytest.mark.parametrize("name", ["hello", "paper1", "world192", "ecoli", "fib", "english", "dna", "uniform8"])
 def test_device_built_tables_match_host_construction(ctx, name):
     """hb_build_tables_kernel (one thread per table entry, walking the uploaded node array)
     against csrc/hb_lut.c's host construction, entry by entry"""
-    if name in ("fib", "english"):
-        tree = hb.Model(hb.MODEL_FIBONACCI if name == "fib" else hb.MODEL_ENGLISH).tree
+    models = {"fib": hb.MODEL_FIBONACCI, "english": hb.MODEL_ENGLISH, "dna": hb.MODEL_DNA, "uniform8": hb.MODEL_UNIFORM8}
+    if name in models:
+        tree = hb.Model(models[name]).tree
     else:
         tree = _stream(name).tree
     lut = hb.build_lut(tree)
@@ -492,7 +508,7 @@ def test_tree_with_more_than_256_internal_nodes(ctx, dev):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("geom", [(0, -1), (8, 4), (10, 4), (11, 3), (12, 2), (12, 0), (9, 1)])
-@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "ecoli", "bible"])
+@pytest.mark.parametrize("name", ["paper1", "world192", "kjv", "ecoli", "bible", "english4m", "dna4m", "fib1m", "uniform1m"])
 def test_flat_emit_table_geometries(dev, name, geom):
     """hb_emitf_kernel with every EP-table shape (index bits, log2 copies): same bytes, at
     several output alignments; nothing written outside the slice"""
@@ -503,7 +519,7 @@ def test_flat_emit_table_geometries(dev, name, geom):
     cb = hb.Codebook(c, f.tree)
     for off in (0, 1, 6, 11):
         got, res, raw = _decode_dev(c, cb, f, dev, out_offset=off)
-        assert res["n_symbols"] == f.usize and O.sha256(got) == O.CORPORA[name][2], (geom, off)
+        assert res["n_symbols"] == f.usize and O.sha256(got) == O.digest(name), (geom, off)
         assert not raw[off + f.usize:].any() and not raw[:off].any()
     cb.close()
     c.close()

@@ -71,8 +71,8 @@ def test_container_round_trip_both_widths(tmp_path):
         assert g.wide == wide and (g.nodes, g.bits, g.usize) == (f.nodes, f.bits, f.usize)
         assert np.array_equal(g.tree, f.tree) and np.array_equal(g.data[: g.nbytes], f.data[: f.nbytes])
         assert np.array_equal(O.load_huff(p).data[: g.nbytes], f.data[: f.nbytes])   # oracle reads HUF8 too
-    if O.ref() is not None:   # the v1 writer is byte-identical to the shipped file
-        assert open(str(tmp_path / "x0.huff"), "rb").read() == open(os.path.join(O.GOLDEN_DIR, "paper1.huff"), "rb").read()
+    # the v1 writer is byte-identical to the shipped file
+    assert open(str(tmp_path / "x0.huff"), "rb").read() == open(os.path.join(O.GOLDEN_DIR, "paper1.huff"), "rb").read()
     with pytest.raises(hb.HuffError):
         hb.HuffFile.load(os.path.join(O.GOLDEN_DIR, "paper1"))   # plaintext is not a .huff
     with pytest.raises(hb.HuffError):
