@@ -769,6 +769,63 @@ HB_HD hb_tail hb_emit_words32(const hb_tables32 &tb, const uint32_t (&w)[WPT + 1
     return hb_w32_tail(st);
 }
 
+/* hb_push32 that also keeps the staging word it stores in `last` */
+HB_HD uint32_t hb_push32_keep(uint32_t ent, uint32_t t, uint32_t &pend, uint32_t posk, hb_out_t &wpp,
+                              uint32_t &last) {
+    const uint32_t word = hb_funnel_l(pend, ent, posk);
+    const uint32_t posk_n = posk + t;
+    pend = hb_funnel_r(pend, ent, t);
+    if ((posk ^ posk_n) & 0x20u) { hb_st32(wpp, 0u, word); wpp += 4; last = word; }
+    return posk_n;
+}
+
+/* Whole chain of a FULL subsequence with an unclipped end (hb_emit32w_kernel's one-window path).
+ * The last word runs the plain probe loop until the position leaves the word.  The last probe starts
+ * inside the subsequence, so its first codeword is this chain's; the at most HB_E32_MAXSYM - 1 symbols
+ * behind it are the right neighbour's first ones, decoded right because the chain is synchronised.
+ * Those two bytes can complete at most one staging word: the one holding this chain's last byte, the
+ * "boundary word".  The right neighbour's first store writes the same word with zeros where this
+ * chain's bytes go, and the two stores land in either order.  So the returned tail holds this chain's
+ * k = (out + c) & 3 bytes of the boundary word, to be stored once more after the warp's barrier
+ * (hb_store_tail): from the pending bytes, or from the last word stored when the overrun completed the
+ * boundary word.  A full subsequence starts at least S / HB_MAX_CODELEN >= 8 codewords, so every
+ * chain completes its own first word and no two chains share a boundary word. */
+template <int WPT, bool ADD = false>
+HB_HD hb_tail hb_emit_words32_run(const hb_tables32 &tb, const uint32_t (&w)[WPT + 1], uint32_t e,
+                                  uint32_t c, hb_out_t out, uint32_t mis) {
+    const uint32_t SC = tb.sc;
+    uint32_t acc = e, pend = 0u, posk = 8u * mis, last = 0u;
+    hb_out_t wpp = out - mis;
+#pragma unroll
+    for (int j = 0; j < WPT; j++) {
+        const uint32_t lo = w[j], hi = w[j + 1];
+        const uint32_t los = hb_keep(lo << SC), his = hb_funnel_l(lo, hi, SC);
+        for (;;) {
+            do {
+                const uint32_t ent = hb_probe32<ADD>(tb, los, his, acc);
+                if (j == WPT - 1) posk = hb_push32_keep(ent, hb_e32_shift(ent), pend, posk, wpp, last);
+                else posk = hb_push32(ent, hb_e32_shift(ent), pend, posk, wpp);
+                acc = hb_e32_advance(acc, ent);
+            } while (!(acc & 0xE0u));
+            if (acc < HB_E64_MARK) break;
+            acc -= HB_E64_MARK;
+            const uint32_t ent = hb_e32_single(tb.slow, lo, hi, acc);
+            if (j == WPT - 1) posk = hb_push32_keep(ent, 8u, pend, posk, wpp, last);
+            else posk = hb_push32(ent, 8u, pend, posk, wpp);
+            acc = hb_e32_advance(acc, ent);
+            if (acc & 0xE0u) break;
+        }
+        acc -= 32u;
+    }
+    /* d: this chain's bytes from the pending word's start, in [-2, 3] (the overrun is at most 2 bytes) */
+    const int32_t d = (int32_t)c - (int32_t)(wpp - out);
+    const uint32_t np = (posk >> 3) & 3u;
+    hb_tail tl;
+    if (d >= 0) { tl.k = (uint32_t)d; tl.at = wpp; tl.bytes = pend >> ((32u - 8u * np) & 31u); }
+    else { tl.k = (uint32_t)(d + 4); tl.at = wpp - 4; tl.bytes = last; }
+    return tl;
+}
+
 /* Partial subsequence (stream tail): byte stores, every symbol clipped to the chain's count c */
 template <int WPT, bool ADD = false>
 HB_HD uint32_t hb_emit_clipped32(const hb_tables32 &tb, const uint32_t (&w)[WPT + 1], uint32_t lim,

@@ -1360,6 +1360,39 @@ hb_emit32w_kernel(hb_stream_args a, uint32_t rshift, uint32_t tab_off, uint32_t 
         }
         const uint32_t o = inc - c;
         const uint64_t Bt = B + front;
+        if constexpr (!E64 && SPL == 1) {
+            /* The common case, compiled on its own: the warp tile's output fits one window, and it is not in
+             * the shard's last sync tile, so every subsequence is whole and every symbol valid.  The chains
+             * end unclipped (hb_emit_words32_run); the window is [al, al + nk) of the slice. */
+            if (nk <= win && u + WT < nunits && cap_ok) {
+                const uint32_t al = (uint32_t)((reinterpret_cast<uintptr_t>(out) + Bt) & 15u);
+                if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                __syncwarp();
+                const hb_out_t dst = (hb_out_t)(s_out_saddr + al + o);
+                const hb_tail tl = hb_emit_words32_run<WPT, ADD>(tb, w, e, c, dst, (uint32_t)(uintptr_t)dst & 3u);
+                advance();
+                if (u < nunits) fetch();
+                __syncwarp();                    /* every right neighbour's first store is done */
+                hb_store_tail(tl);
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                __syncwarp();
+                uint8_t *gbase = out + Bt - al;  /* 16-byte aligned */
+                const uint32_t endb = al + nk, a0 = (al + 15u) & ~15u, a1 = endb & ~15u;
+                if (a0 < a1) {
+                    if (lane == 0) {
+                        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
+                                     :: "l"(gbase + a0), "r"(s_out_saddr + a0), "r"(a1 - a0) : "memory");
+                        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                    }
+                    /* fewer than 16 bytes each: the head on lanes 0-15, the tail on lanes 16-31 */
+                    const uint32_t i = lane < 16u ? al + lane : a1 + (lane - 16u);
+                    if (i < (lane < 16u ? a0 : endb)) gbase[i] = s_out[i];
+                } else if (al + lane < endb) {
+                    gbase[al + lane] = s_out[al + lane];   /* < 32 bytes */
+                }
+                continue;
+            }
+        }
         /* Only in the shard's last sync tile can the stream end inside a subsequence, or the shard's last
          * codeword be cut off (its symbol is then not part of total_valid): everywhere else every
          * subsequence is whole and every symbol valid, and the 64-bit bookkeeping is skipped. */
